@@ -46,6 +46,7 @@ if os.environ.get("NCCL_DEBUG", "").upper() in ("VERSION", "WARN"):
     os.environ["NCCL_DEBUG"] = "NONE"      # the version banner is printed to stdout at these levels
 
 METRIC = "densenet121_cifar10_images_per_sec"
+DUMP_MAX_PARAMS = 15_000_000          # 60 MB of float32: --dump-outputs stays below 64 MB in all
 MODEL_NAMES = {"densenet": "densenet121", "resnet": "resnet101"}
 
 
@@ -75,6 +76,12 @@ def parse():
                    help="own arm: tf32 (default: fp32 storage + TF32 tensor-core math = the precision class of the reference's fp32 "
                         "model with cuDNN's default TF32 convolutions) | bf16 | fp32 | auto")
     p.add_argument("--alt-dtype", default="bf16", help="own arm: additionally measure this dtype and report it under 'alt' ('' = skip)")
+    p.add_argument("--dump-outputs", metavar="DIR", default="",
+                   help="own arm: after the timed steps, write what the last of them computed (headline dtype, rank 0) to "
+                        "DIR/<name>.npy: loss.npy = that step's loss, params.npy = the updated parameters, flattened in "
+                        "named_parameters() order (a fixed, seeded sample when there are more than DUMP_MAX_PARAMS).  "
+                        "That step starts from the initial training state, so its outputs depend on the arguments and the "
+                        "build only")
     return p.parse_args()
 
 
@@ -185,6 +192,18 @@ def common_config(a, world, is_lm, throttle, rounds, W):
     return cfg
 
 
+def dump_outputs(out_dir: str, model, step_loss) -> None:
+    """What a caller of the training step receives from the last timed step: its loss and the updated parameters."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "loss.npy"), step_loss.detach().float().cpu().numpy())
+    params = torch.cat([p.detach().float().reshape(-1) for p in model.parameters()]).cpu().numpy()
+    if params.size > DUMP_MAX_PARAMS:
+        params = params[np.sort(np.random.RandomState(0).choice(params.size, DUMP_MAX_PARAMS, replace=False))]
+    np.save(os.path.join(out_dir, "params.npy"), params)
+
+
 # =====================================================================================================
 def run_ours(a) -> dict:
     if ROOT not in sys.path:
@@ -210,7 +229,7 @@ def run_ours(a) -> dict:
         a.dataset = "wikitext2"
     clocks = ClockSampler(local)
 
-    def measure(dtype: str) -> dict:
+    def measure(dtype: str, dump_dir: str = "") -> dict:
         S = max(3, a.dbs_steps)
         total_steps = rounds * S + W + 2 * K + 8
         extra = {} if a.dbs_model == "auto" else {"dbs_model": a.dbs_model}
@@ -224,6 +243,9 @@ def run_ours(a) -> dict:
         logger = init_logger(cfg, rank, stream=False)
         tr = Trainer(cfg, rank, world, device, logger)
         is_lm = tr.is_lm
+        if dump_dir:
+            state = [t for t in (tr.flat.master, tr.flat.mom, tr.flat.shadow) if t is not None]
+            initial_state = [t.clone() for t in state]
 
         def make_shard(local_batches, n_steps, seed):
             if is_lm:
@@ -244,7 +266,8 @@ def run_ours(a) -> dict:
                 lm_cache[key] = batchify(stream[off:off + need], b).pin_memory()
             return lm_cache[key]
 
-        def run_steps(shard, n, e2e=True, sink=None):
+        def run_steps(shard, n, e2e=True, sink=None, before_last=None):
+            """``before_last``: called just before the last step is issued"""
             import numpy as np
             if is_lm:
                 b, n_steps, seed = shard
@@ -254,6 +277,8 @@ def run_ours(a) -> dict:
                     if e2e or s == 0:
                         src = data[i:i + cfg.bptt].to(device, non_blocking=True)                  # H2D from pinned memory
                         tgt = data[i + 1:i + 1 + cfg.bptt].reshape(-1).to(device, non_blocking=True)
+                    if before_last is not None and s == n - 1:
+                        before_last()
                     tr.train_step(src, tgt)
                     if e2e and sink is not None:
                         sink[s % sink.shape[0]].copy_(tr.loss_acc, non_blocking=True)
@@ -262,6 +287,8 @@ def run_ours(a) -> dict:
             for s in range(n):
                 if e2e or s == 0:
                     xb, yb = tr.stager.stage(shard.batch_indices(s, order))
+                if before_last is not None and s == n - 1:
+                    before_last()
                 tr.train_step(xb, yb)
                 if e2e:
                     tr.stager.release()
@@ -294,7 +321,7 @@ def run_ours(a) -> dict:
         torch.cuda.synchronize()
         sink = torch.zeros(8, 1, dtype=torch.float32).pin_memory()
 
-        def timed(e2e: bool, seed: int):
+        def timed(e2e: bool, seed: int, before_last=None):
             shard = make_shard(lb, K, seed)
             if world > 1:
                 dist.barrier()
@@ -306,7 +333,7 @@ def run_ours(a) -> dict:
             e0.record()
             h0 = time.perf_counter()
             blocked0 = tr.stager.blocked_s if tr.stager is not None else 0.0
-            run_steps(shard, K, e2e=e2e, sink=sink if e2e else None)
+            run_steps(shard, K, e2e=e2e, sink=sink if e2e else None, before_last=before_last)
             host_ms = (time.perf_counter() - h0) * 1e3          # wall time of the issuing loop, including ...
             # ... back-pressure: with a 4-deep staging ring the host blocks once it is 4 steps ahead of the device
             host_ms -= ((tr.stager.blocked_s if tr.stager is not None else 0.0) - blocked0) * 1e3
@@ -320,7 +347,19 @@ def run_ours(a) -> dict:
             return max_over_ranks(ms, device, world), _native.launch_count() - n0, max_over_ranks(wait, device, world), host_ms
 
         ms_e2e, _, wait_e2e, host_e2e = timed(True, 3)
-        ms_dev, launches, wait_dev, host_dev = timed(False, 4)
+        restart = None
+        if dump_dir:
+            loss_before_last = torch.zeros_like(tr.loss_acc)
+
+            def restart():
+                # the kernels accumulate with float atomics, so run-to-run rounding differences compound from step to step;
+                # the dumped step starts from the initial state instead (device copies, in stream order with the steps)
+                for dst, src in zip(state, initial_state):
+                    dst.copy_(src)
+                loss_before_last.copy_(tr.loss_acc)
+        ms_dev, launches, wait_dev, host_dev = timed(False, 4, restart)
+        if dump_dir and rank == 0:
+            dump_outputs(dump_dir, tr.model, tr.loss_acc - loss_before_last)
         if hasattr(tr.comm, "check_errors"):
             tr.comm.check_errors()
         per_step_items = a.batch * (cfg.bptt if is_lm else 1)          # images, or tokens for the LM
@@ -340,7 +379,7 @@ def run_ours(a) -> dict:
 
     if rank == 0:
         clocks.start()
-    main_res = measure(a.dtype)
+    main_res = measure(a.dtype, a.dump_outputs)
     clk = clocks.stop() if rank == 0 else {}
     alt = None
     if a.alt_dtype and a.alt_dtype != a.dtype:

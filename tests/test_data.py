@@ -9,7 +9,7 @@ import torch
 from dynamic_load_balance_distributeddnn_b200.data import (Corpus, DataPartitioner, batchify, get_batch,
                                                             global_permutation, load_corpus, load_image_dataset,
                                                             split_token_stream)
-from dynamic_load_balance_distributeddnn_b200.data.corpus import SyntheticCorpus
+from dynamic_load_balance_distributeddnn_b200.data.corpus import WIKITEXT2_TOKENS, WIKITEXT2_VOCAB, SyntheticCorpus
 from dynamic_load_balance_distributeddnn_b200 import ops
 
 
@@ -64,10 +64,19 @@ def test_corpus_tokenize(tmp_path):
     assert s.ntokens == 100 and int(s.train.max()) == 99
 
 
-@pytest.mark.skipif(not os.path.isfile("/root/reference/rnn_data/wikitext-2/train.txt"), reason="corpus not mounted")
-def test_wikitext2_vocab():
-    c = load_corpus("/root/reference/rnn_data/wikitext-2")
-    assert c.ntokens == 33278 and c.train.numel() == 2088628 and c.valid.numel() == 217646 and c.test.numel() == 245569
+def test_wikitext2_vocab(monkeypatch, tmp_path):
+    """tests/golden/wikitext2_sample holds the first lines of each wikitext-2 split; wikitext2_sample.npz the token ids and
+    vocabulary size the reference's Corpus produced for them, and its vocabulary size and split lengths on the full corpus
+    (the shape the synthetic stand-in copies)."""
+    golden = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+    ref = np.load(os.path.join(golden, "wikitext2_sample.npz"))
+    monkeypatch.setenv("DLB_CACHE_DIR", str(tmp_path))
+    c = load_corpus(os.path.join(golden, "wikitext2_sample"))
+    assert c.ntokens == int(ref["ntokens"])
+    for split in ("train", "valid", "test"):
+        assert getattr(c, split).tolist() == ref[split].tolist(), split
+    full = ref["full"].tolist()
+    assert full == [WIKITEXT2_VOCAB, WIKITEXT2_TOKENS["train"], WIKITEXT2_TOKENS["valid"], WIKITEXT2_TOKENS["test"]]
 
 
 def test_synthetic_images_and_augment():

@@ -3,11 +3,13 @@ into the flat symmetric buffer) and the precision modes (bf16 / tf32) of a full 
 import math
 import os
 
+import numpy as np
 import pytest
 import torch
 import torch.nn.functional as F
 
 pytestmark = pytest.mark.gpu
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "gradpath.npz")
 
 
 @pytest.fixture(scope="module")
@@ -79,41 +81,61 @@ def test_gradient_sinks_match_pack_path(nat, tmp_path):
     a.close(); b.close()
 
 
-@pytest.mark.parametrize("dtype,tol", [("tf32", 2e-2), ("bf16", 0.15)])
-def test_densenet_step_matches_fp32_torch_model(nat, tmp_path, dtype, tol):
-    """one full optimisation step (augment off) of the native DenseNet-121 vs the same step done with plain torch.nn ops in
-    fp32 on the same weights: loss and parameter update."""
-    torch.backends.cudnn.allow_tf32 = False
-    torch.backends.cuda.matmul.allow_tf32 = False
-    t = _trainer(tmp_path, dtype, dtype=dtype, bs=16)
-    # the reference's own DenseNet-121 (stock torch.nn layers), loaded by file path from the installed reference
-    import importlib.util
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    path = os.path.join(root, "baseline", "_ref", "Net", "Densenet.py")
-    if not os.path.isfile(path):
-        pytest.skip("baseline/_ref not installed")
-    spec = importlib.util.spec_from_file_location("_ref_densenet", path)
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    ref = mod.DenseNet121(10).cuda().float()
-    sd = {k: v.detach().float().clone() for k, v in t.model.state_dict().items()}
-    ref.load_state_dict(sd)
+def gradient_sample(numels, budget=1024, seed=0):
+    """Stratified sample of a model's parameters: every tensor gets a share of ``budget`` proportional to its size (at least
+    one element).  Returns (tensor index, element index) arrays."""
+    rng = np.random.RandomState(seed)
+    total = sum(numels)
+    ti, ei = [], []
+    for i, n in enumerate(numels):
+        k = min(n, max(1, round(budget * n / total)))
+        ti.append(np.full(k, i))
+        ei.append(np.sort(rng.choice(n, k, replace=False)))
+    return np.concatenate(ti), np.concatenate(ei)
+
+
+def _flat_sample(params, ti, ei):
+    return torch.cat([p.detach().float().reshape(-1)[torch.as_tensor(ei[ti == i], device=p.device)]
+                      for i, p in enumerate(params)]).cpu().numpy()
+
+
+def _step_matches_reference(t, case, tol):
+    """One optimisation step (augment off) of trainer ``t`` on images 0..15 vs the reference model's fp32 step on the same
+    weights and images, recorded under tests/golden/ by tools/make_golden.py: the loss, and the relative L2 distance of the
+    update / lr (= the gradient: first step, empty momentum buffer) from the reference gradient, estimated on a stratified
+    sample of every parameter tensor."""
+    gold = np.load(GOLDEN)
+    pre = case + "/"
+    params = [p for _, p in t.model.named_parameters()]
+    numel = np.array([p.numel() for p in params])
+    assert numel.tolist() == gold[pre + "numel"].tolist(), "parameter layout differs from the recorded reference model"
+    ti, ei = gradient_sample(numel.tolist())
     xb, yb = t.stager.stage(list(range(16)))
-    x = t._prepare_images(xb).float()
-    before = {k: v.detach().float().clone() for k, v in t.model.named_parameters()}
-    out = ref(x.contiguous())
-    loss_ref = F.cross_entropy(out, yb)
-    loss_ref.backward()
+    x = t._prepare_images(xb).double()
+    assert yb.tolist() == gold[pre + "labels"].tolist()
+    assert abs(x.sum().item() - float(gold[pre + "x_sum"])) < 1e-4 * x.abs().sum().item(), "inputs differ from the recording"
+    before = _flat_sample(params, ti, ei)
+    np.testing.assert_allclose(before, gold[pre + "w0"], rtol=1e-6, atol=1e-7, err_msg="initial weights differ from the recording")
     t.train_step(xb, yb)
     t.stager.release()
     torch.cuda.synchronize()
-    assert abs(t.loss_acc.item() - loss_ref.item()) < tol * max(1.0, loss_ref.item()), (t.loss_acc.item(), loss_ref.item())
-    num = den = 0.0
-    for (k, p), (_, pr) in zip(t.model.named_parameters(), ref.named_parameters()):
-        upd = (before[k] - p.detach().float()) / 0.05           # = gradient (first step, momentum buffer empty)
-        num += (upd - pr.grad).pow(2).sum().item()
-        den += pr.grad.pow(2).sum().item()
-    assert math.sqrt(num / den) < tol * 3, math.sqrt(num / den)
+    loss_ref = float(gold[pre + "loss"])
+    assert abs(t.loss_acc.item() - loss_ref) < tol * max(1.0, loss_ref), (t.loss_acc.item(), loss_ref)
+    upd = (before - _flat_sample(params, ti, ei)) / 0.05
+    g = gold[pre + "grad"]
+    w = (numel / np.bincount(ti, minlength=len(numel)))[ti]       # stratum weight of each sampled element
+    rel = math.sqrt(float((w * (upd - g) ** 2).sum() / (w * g ** 2).sum()))
+    assert rel < 3 * tol, rel
+
+
+@pytest.mark.parametrize("dtype,tol", [("tf32", 2e-2), ("bf16", 0.15)])
+def test_densenet_step_matches_fp32_torch_model(nat, tmp_path, dtype, tol):
+    """one full optimisation step (augment off) of the native DenseNet-121 vs the same step of the reference's own
+    DenseNet-121 (stock torch.nn layers, fp32) on the same weights: loss and parameter update."""
+    torch.backends.cudnn.allow_tf32 = False
+    torch.backends.cuda.matmul.allow_tf32 = False
+    t = _trainer(tmp_path, dtype, dtype=dtype, bs=16)
+    _step_matches_reference(t, "densenet-" + dtype, tol)
     t.close()
 
 
@@ -142,33 +164,10 @@ def test_tf32_training_decreases_loss_like_bf16(nat, tmp_path):
     ("regnet", "RegNet", "RegNetY_400MF", "tf32", 3e-2)])
 def test_family_step_matches_reference_model(nat, tmp_path, model, ref_mod, ref_cls, dtype, tol):
     """Full optimisation step of a zoo family through the native kernels (GN fusions, tcgen05 convs, SE / stem kernels, flat
-    optimizer) vs the REFERENCE's own class (stock torch.nn, true fp32) on the same weights: loss + relative L2 of the update."""
-    import importlib.util
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    path = os.path.join(root, "baseline", "_ref", "Net", ref_mod + ".py")
-    if not os.path.isfile(path):
-        pytest.skip("baseline/_ref not installed")
+    optimizer) vs the REFERENCE's own class ``ref_mod.ref_cls`` (stock torch.nn, true fp32) on the same weights: loss +
+    relative L2 of the update."""
     torch.backends.cudnn.allow_tf32 = False
     torch.backends.cuda.matmul.allow_tf32 = False
     t = _trainer(tmp_path, model + dtype, dtype=dtype, model=model, bs=16)
-    spec = importlib.util.spec_from_file_location("_ref_" + ref_mod, path)
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    ref = getattr(mod, ref_cls)(10).cuda().float()
-    ref.load_state_dict({k: v.detach().float().clone() for k, v in t.model.state_dict().items()})
-    xb, yb = t.stager.stage(list(range(16)))
-    x = t._prepare_images(xb).float()
-    before = {k: v.detach().float().clone() for k, v in t.model.named_parameters()}
-    loss_ref = F.cross_entropy(ref(x.contiguous()), yb)
-    loss_ref.backward()
-    t.train_step(xb, yb)
-    t.stager.release()
-    torch.cuda.synchronize()
-    assert abs(t.loss_acc.item() - loss_ref.item()) < tol * max(1.0, loss_ref.item()), (t.loss_acc.item(), loss_ref.item())
-    num = den = 0.0
-    for (k, p), (_, pr) in zip(t.model.named_parameters(), ref.named_parameters()):
-        upd = (before[k] - p.detach().float()) / 0.05
-        num += (upd - pr.grad).pow(2).sum().item()
-        den += pr.grad.pow(2).sum().item()
-    assert math.sqrt(num / den) < 3 * tol, math.sqrt(num / den)
+    _step_matches_reference(t, f"{model}-{dtype}", tol)
     t.close()
